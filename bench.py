@@ -71,7 +71,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the strong_scaling and extra.workloads blocks")
     ap.add_argument("--h2d-chunks", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0's visits, root values, ...) as DIR/<name>.npy; the inputs "
+                         "are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     select_workload(args.workload)
     args.roots = args.roots or ROOTS_PER_GPU
     args.sims = args.sims or NUM_SIMULATIONS
@@ -221,6 +228,26 @@ class ClockSampler:
 # ------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, result):
+    """Writes the per-root arrays of one search_batch result as out_dir/<name>.npy in float32 (visit counts are exact there).
+    When together they would pass DUMP_LIMIT bytes, the same seeded sample of roots is taken from each and its root
+    indices are written as rows.npy."""
+    import numpy as np
+    arrays = {k: v.cpu().numpy().astype(np.float32) for k, v in result.items()}
+    roots = len(arrays["visits"])
+    row_bytes = sum(a[0].nbytes for a in arrays.values())
+    if roots * row_bytes > DUMP_LIMIT:
+        rows = np.sort(np.random.default_rng(0).choice(roots, (DUMP_LIMIT - 4096) // (row_bytes + 8), replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def _peak():
     pk_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(pk_path):
@@ -322,6 +349,7 @@ def ours(args, rank, local_rank, world):
             r = w["policy"].search_batch(w["d_f32"][i % w["NBUF"]], w["d_mask"], w["d_noise"], None, deterministic=True, read_back=False)
             if world > 1 and gather:   # the only collective of the path: all-gather of the finished results over NCCL
                 gather_search_results(r["visits"], r["values"], w["B"] * world)
+            w["last"] = r
             return r
         return fn
 
@@ -376,6 +404,8 @@ def ours(args, rank, local_rank, world):
         time.sleep(0.3)
     dev_ms, wall_ms, launches = timed(device_step(W), args.steps, warm)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:     # before the e2e steps reuse the policy's output buffers
+        dump_outputs(args.dump_outputs, W["last"])
     e2e_dev_ms, e2e_wall_ms, _ = timed(e2e_step(W), args.steps, warm)
     e2e_full_wall_ms = e2e_wall_ms
     if W["fs"] is not None:

@@ -253,6 +253,25 @@ def make_case_reuse(mod, B, A, S, masks, noise, two_player, scale, seed, horizon
                 discount=np.float32(DISCOUNT), delta=np.float32(DELTA), noise_w=np.float32(NOISE_W), lstm_horizon_len=horizon)
 
 
+def record_random_runs(mz, ez, mz_rand0):
+    """tests/golden/ref_random_runs.json.gz: the compiled reference's results of every random run test_oracle_pin.py compares
+    the C port against (RANDOM_RUNS there), each run twice to show the record is reproducible."""
+    import gzip
+    import json
+    sys.path.insert(0, os.path.dirname(HERE))
+    from test_oracle_pin import RANDOM_RUNS, random_run_cases, summarize_run
+    mods = {"mz": mz, "ez": ez, "reuse_mz": mz_rand0, "reuse_ez": ez}
+    rec = {}
+    for tree, (run, seeds, _) in RANDOM_RUNS.items():
+        for seed in seeds:
+            for key, args in random_run_cases(tree, seed):
+                rec[key] = summarize_run(run(mods[tree], False, *args))
+                assert summarize_run(run(mods[tree], False, *args)) == rec[key], key
+    with gzip.GzipFile(os.path.join(HERE, "ref_random_runs.json.gz"), "wb", compresslevel=9, mtime=0) as f:
+        f.write(json.dumps(rec, sort_keys=True, separators=(",", ":")).encode())
+    print("random runs recorded:", len(rec))
+
+
 def main():
     import mz_tree
     for name, *args in CASES:
@@ -289,6 +308,7 @@ def main():
         np.savez_compressed(os.path.join(HERE, f"{name}.npz"), **case)
         print(name, "sum visits ok:", bool((np.where(case["distributions"] < 0, 0, case["distributions"]).sum(1) == case["S"]).all()),
               "no-inference marks:", int((case["ix"] == -1).sum()))
+    record_random_runs(mz_tree, ez_tree, mz_rand0)
 
 
 if __name__ == "__main__":
