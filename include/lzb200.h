@@ -141,6 +141,32 @@ int lz_tree_backpropagate_with_reuse(lz_tree *t, int latent_index, const float *
 int lz_tree_select_action(lz_tree *t, float temperature, int deterministic, uint64_t seed, int32_t *d_action,
                           int32_t *d_action_pos, float *d_entropy, lz_stream s);
 
+/* ---- Gumbel MuZero tree (lzero/mcts/ctree/ctree_gumbel_muzero/lib/cnode.cpp, gmz_tree.pyx) ----
+ * lz_tree_set_gumbel switches a tree to Gumbel mode (before lz_tree_prepare_gumbel) and precomputes on the host the fixed
+ * Gumbel draw (std::mt19937(0), 10 * extreme_value(0, 1), cnode.cpp:1133-1151; every root uses the prefix of its legal-list
+ * length) and the considered-visit row get_sequence_of_considered_visits(min(m, S), S) (:1041-1094).  Root choice is
+ * sequential halving (cselect_root_child, :701-745), interior choice the completed-Q improved policy (cselect_interior_child,
+ * :747-790).  Nothing on the search path draws random numbers: every call reproduces the reference bit for bit.
+ * LZ_EINVAL when num_simulations exceeds the tree's max_sims. */
+int lz_tree_set_gumbel(lz_tree *t, int num_simulations, int max_num_considered_actions);
+/* CRoots::prepare / prepare_no_noise (cnode.cpp:418-455): lz_tree_prepare plus the root's raw value d_values f32 [B] (NULL: 0). */
+int lz_tree_prepare_gumbel(lz_tree *t, const float *d_logits, const float *d_noise, float noise_weight,
+                           const float *d_rewards, const float *d_values, const int32_t *d_to_play, lz_stream s);
+/* cbatch_traverse (cnode.cpp:834-897); outputs as lz_tree_traverse, d_virtual_to_play = the root to_play unchanged.
+ * LZ_ESTATE for more than num_simulations traverses since the last prepare (the reference indexes past its table). */
+int lz_tree_traverse_gumbel(lz_tree *t, float discount, int32_t *d_ix, int32_t *d_iy, int32_t *d_last_action,
+                            int32_t *d_search_len, int32_t *d_virtual_to_play, lz_stream s);
+/* cbatch_back_propagate (cnode.cpp:605-652): expand the leaves into slot latent_index, store d_value as their raw value, back up
+ * (single-player recurrence for every to_play: the reference asserts to_play == -1 and is built with NDEBUG). */
+int lz_tree_backpropagate_gumbel(lz_tree *t, int latent_index, float discount, const float *d_reward,
+                                 const float *d_value, const float *d_logits, lz_stream s);
+/* get_children_values (cnode.cpp:309-338) -> d_children_values f32 [B,A] by action id, -inf for illegal actions;
+ * get_policies (:355-385) -> d_improved_policy f32 [B,A] by action id, illegal entries 0;
+ * d_action int32 [B]: np.argmax of the improved policy with illegal entries 0 (gumbel_muzero.py:591-592).  Any may be NULL.
+ * Visit counts, root values and trajectories come from lz_tree_results. */
+int lz_tree_results_gumbel(lz_tree *t, float discount, float *d_children_values, float *d_improved_policy,
+                           int32_t *d_action, lz_stream s);
+
 /* ------------------------------------------------------------------ model (muzero_model.py, efficientzero_model.py) */
 
 typedef struct lz_model_config {
@@ -240,6 +266,11 @@ int lz_search_run_ez(lz_search *q, const float *d_latent_roots, const float *d_h
  * tree at :1040-1046 / cnode.cpp:646, see DESIGN.md 4.6). */
 int lz_search_run_ez_with_reuse(lz_search *q, const float *d_latent_roots, const float *d_hidden0_roots, const float *d_hidden1_roots,
                                 const int32_t *d_true_action, const float *d_reuse_value, int32_t *d_infer_count, lz_stream s);
+/* GumbelMuZeroMCTSCtree.search (mcts_ctree.py:1076-1174) on roots prepared with lz_tree_prepare_gumbel, for a search created
+ * from a MuZero model (conv or MLP) and a tree set to Gumbel mode with num_simulations equal to the search's.  One CUDA graph
+ * [traverse] + S x [recurrent_inference, backpropagate (+ next traverse)], re-captured when the weights, the tree's Gumbel
+ * parameters or the discount change. */
+int lz_search_run_gumbel(lz_search *q, const float *d_latent_roots, float discount, lz_stream s);
 /* The search-feeding part of _forward_collect (policy/muzero.py:749-779): initial_inference ->
  * reset(mask) -> prepare(noise) -> search.  d_obs f32 [B,obs_c,H,W]; d_mask uint8 [B,A] or NULL;
  * d_noise f32 [B,A] legal-order rows or NULL; d_to_play int32 [B] or NULL (-1).

@@ -1,7 +1,7 @@
 """Builds lightzero_b200/_lib/liblzb200.so (the C-ABI library, include/lzb200.h) with nvcc for sm_100a.
 
 In-tree build: the .so is git-ignored but travels to the GPU box with the gpurun snapshot.
-tree.cu is compiled with -fmad=false (the reference tree is built for baseline x86-64 and never
+tree.cu and gumbel.cu are compiled with -fmad=false (the reference tree is built for baseline x86-64 and never
 contracts a*b+c; bit-exact visit counts depend on it); the network kernels want FMA.
 """
 import os
@@ -16,7 +16,7 @@ ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler", "-fno-fast-math"]
 # Experiment builds: `python -m lightzero_b200._build --tag NAME -DFOO ...` writes _lib/NAME/liblzb200.so with the extra
 # defines; LZ_LIB_TAG=NAME makes cabi.load() pick it (one GPU session can then compare several kernel variants).
-UNITS = [("tree.cu", ["-fmad=false"]), ("model.cu", []), ("net_tc.cu", []), ("conv_tc.cu", []), ("mlp.cu", []), ("ez.cu", []), ("search.cu", []), ("collector.cu", [])]
+UNITS = [("tree.cu", ["-fmad=false"]), ("gumbel.cu", ["-fmad=false"]), ("model.cu", []), ("net_tc.cu", []), ("conv_tc.cu", []), ("mlp.cu", []), ("ez.cu", []), ("search.cu", []), ("collector.cu", [])]
 
 
 def _stale(target, deps):

@@ -52,6 +52,11 @@ SIGNATURES = {
     "lz_tree_traverse_ez": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "lz_tree_backpropagate_ez": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "lz_tree_results": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "lz_tree_set_gumbel": (c_int, [c_void_p, c_int, c_int]),
+    "lz_tree_prepare_gumbel": (c_int, [c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "lz_tree_traverse_gumbel": (c_int, [c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "lz_tree_backpropagate_gumbel": (c_int, [c_void_p, c_int, c_float, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "lz_tree_results_gumbel": (c_int, [c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p]),
     "lz_model_create": (c_int, [ctypes.POINTER(ModelConfig), ctypes.POINTER(c_void_p)]),
     "lz_model_create_mlp": (c_int, [ctypes.POINTER(MlpConfig), ctypes.POINTER(c_void_p)]),
     "lz_model_destroy": (c_int, [c_void_p]),
@@ -82,6 +87,7 @@ SIGNATURES = {
     "lz_search_num_kernels": (c_int, [c_void_p]),
     "lz_search_latent_pool": (c_void_p, [c_void_p]),
     "lz_search_run_with_reuse": (c_int, [c_void_p] * 6),
+    "lz_search_run_gumbel": (c_int, [c_void_p, c_void_p, c_float, c_void_p]),
     "lz_search_run_ez": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "lz_search_run_ez_with_reuse": (c_int, [c_void_p] * 8),
     "lz_frames_create": (c_int, [c_int, c_int, c_int, c_int, ctypes.POINTER(c_void_p)]),

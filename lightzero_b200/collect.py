@@ -213,3 +213,94 @@ class EfficientZeroCollectPolicy(MuZeroCollectPolicy):
         self.mcts = EfficientZeroMCTSCtree(cfg or {})
         self.cfg = self.mcts._cfg
         self._tree_mode = (1, int(self.cfg.lstm_horizon_len))
+
+
+class GumbelMuZeroCollectPolicy:
+    """``GumbelMuZeroPolicy._forward_collect`` / ``_forward_eval`` (lzero/policy/gumbel_muzero.py:520-607, 619-705): initial
+    inference, roots prepared with the predicted values, the Gumbel search (one CUDA graph with a ``lightzero_b200`` model) and
+    the per-environment output dict.  Everything stays on the device until ONE read-back per step: the action (arg-max of
+    the improved policy with illegal entries 0, :591-592, computed by ``lz_tree_results_gumbel``), the visit counts, the
+    visit-count entropy (``lz_tree_select_action``), the searched value, the completed values (0 off the legal list), the
+    improved policy, the predicted value and the policy logits."""
+
+    def __init__(self, model, cfg: Optional[dict] = None):
+        from .mcts_ctree import GumbelMuZeroMCTSCtree
+        self.model = model
+        self.mcts = GumbelMuZeroMCTSCtree(cfg or {})
+        self.cfg = self.mcts._cfg
+        self.device = model.device
+
+    def _step(self, data, action_mask, noises, to_play, temperature):
+        from . import gmz_tree
+        action_mask = np.asarray(action_mask)
+        B, A = action_mask.shape
+        dev = self.device
+        self.mcts._make_inverse_transforms(dev)
+        with torch.no_grad(), torch.cuda.device(dev):
+            out = self.model.initial_inference(data.to(dev, non_blocking=True))
+            pred = self.mcts._inv(out.value).reshape(-1).contiguous()              # gumbel_muzero.py:546 (inverse transform)
+            roots = gmz_tree.Roots(B, action_mask.astype(np.uint8))
+            if noises is None:
+                roots.prepare_no_noise(None, pred, out.policy_logits, to_play)
+            else:
+                roots.prepare(float(self.cfg.root_noise_weight), noises, None, pred, out.policy_logits, to_play)
+            self.mcts.search(roots, self.model, out.latent_state, to_play)
+            visits, nlegal = roots.get_distributions_tensor()
+            values = roots.get_values_tensor()
+            cv, pol, act = roots.results_tensor(float(self.cfg.discount_factor), A)
+            _, _, ent = roots.select_action_tensor(temperature, deterministic=noises is None)
+            mask = torch.from_numpy(action_mask != 0).to(dev)
+            cv = torch.where(mask, cv, torch.zeros_like(cv))                        # :593
+            flat = torch.cat([act.float(), nlegal.float(), ent, values, pred, visits.float().reshape(-1), cv.reshape(-1),
+                              pol.reshape(-1), out.policy_logits.float().reshape(-1)]).cpu().numpy()   # the one read-back
+            roots.clear()
+        cols = [B, B, B, B, B, B * A, B * A, B * A, B * A]
+        parts = np.split(flat, np.cumsum(cols)[:-1])
+        act, nl, ent, values, pred = parts[:5]
+        visits, cv, pol, logits = (p.reshape(B, A) for p in parts[5:])
+        return act.astype(np.int64), nl.astype(np.int64), ent, values, pred, visits.astype(np.int64), cv, pol, logits
+
+    def forward_collect(self, data: torch.Tensor, action_mask, temperature: float = 1, to_play=(-1,), ready_env_id=None,
+                        **kwargs) -> Dict[int, dict]:
+        """gumbel_muzero.py:520-607: Dirichlet noise over the legal actions (:553-556) drawn with np.random as the reference."""
+        action_mask = np.asarray(action_mask)
+        B, A = action_mask.shape
+        if ready_env_id is None:
+            ready_env_id = np.arange(B)
+        alpha = float(self.cfg.root_dirichlet_alpha)
+        noises = np.zeros((B, A), np.float32)
+        for j in range(B):
+            n = int(action_mask[j].sum())
+            noises[j, :n] = np.random.dirichlet([alpha] * n).astype(np.float32)
+        tp = np.broadcast_to(np.asarray(to_play, np.int32).reshape(-1), (B,)) if np.size(to_play) in (1, B) else np.asarray(to_play)
+        act, nl, ent, values, pred, visits, cv, pol, logits = self._step(data, action_mask, noises, tp.tolist(), temperature)
+        output = {}
+        for i, env_id in enumerate(ready_env_id):
+            output[env_id] = {
+                'action': int(act[i]),
+                'visit_count_distributions': visits[i, :nl[i]].tolist(),
+                'visit_count_distribution_entropy': float(ent[i]),
+                'searched_value': float(values[i]),
+                'roots_completed_value': cv[i],
+                'improved_policy_probs': pol[i],
+                'predicted_value': float(pred[i]),
+                'predicted_policy_logits': logits[i].tolist(),
+            }
+        return output
+
+    def forward_eval(self, data: torch.Tensor, action_mask, to_play=(-1,), ready_env_id=None, **kwargs) -> Dict[int, dict]:
+        """gumbel_muzero.py:619-705: no noise, the same action rule."""
+        action_mask = np.asarray(action_mask)
+        B = action_mask.shape[0]
+        if ready_env_id is None:
+            ready_env_id = np.arange(B)
+        tp = np.broadcast_to(np.asarray(to_play, np.int32).reshape(-1), (B,)) if np.size(to_play) in (1, B) else np.asarray(to_play)
+        act, nl, ent, values, pred, visits, cv, pol, logits = self._step(data, action_mask, None, tp.tolist(), 1.0)
+        return {env_id: {
+            'action': int(act[i]),
+            'visit_count_distributions': visits[i, :nl[i]].tolist(),
+            'visit_count_distribution_entropy': float(ent[i]),
+            'searched_value': float(values[i]),
+            'predicted_value': float(pred[i]),
+            'predicted_policy_logits': logits[i].tolist(),
+        } for i, env_id in enumerate(ready_env_id)}

@@ -88,3 +88,78 @@ LZ_HD float lz_expf_exact(float x)
     return (float)y;
 #endif
 }
+
+// ---- logf -------------------------------------------------------------------------------------------
+// The Gumbel MuZero tree's softmax (ctree_gumbel_muzero/lib/cnode.cpp:903-932) subtracts log(sum) with sum a float,
+// which binds to glibc's logf.  Published algorithm restated: glibc 2.39 sysdeps/ieee754/flt-32/e_logf.c +
+// e_logf_data.c (ARM optimized routines): x = 2^k z with z in [OFF, 2 OFF), a 16-entry table of (1/c, log c) for the
+// subinterval of z, r = z/c - 1 and a degree-3 polynomial for log1p(r), all in double, rounded to float once.
+// Variant: as for expf, glibc's ifunc selects __logf_fma on FMA3 hosts (e_logf.c built with -mfma -ffp-contract=fast),
+// so r = z*invc - 1, y0 = logc + k*Ln2 and the three polynomial steps are fused multiply-adds.
+// tests/csrc/check_logf.c compares this against libm logf on every float in [1, 64] (LZ_EXHAUSTIVE=1: every
+// positive finite float).  Only positive finite inputs are handled (a softmax sum lies in [1, n]); 0 gives -inf.
+#define LZ_LOGF_TAB_INIT { \
+    0x1.661ec79f8f3bep+0, -0x1.57bf7808caadep-2, 0x1.571ed4aaf883dp+0, -0x1.2bef0a7c06ddbp-2, \
+    0x1.49539f0f010bp+0,  -0x1.01eae7f513a67p-2, 0x1.3c995b0b80385p+0, -0x1.b31d8a68224e9p-3, \
+    0x1.30d190c8864a5p+0, -0x1.6574f0ac07758p-3, 0x1.25e227b0b8eap+0,  -0x1.1aa2bc79c81p-3,   \
+    0x1.1bb4a4a1a343fp+0, -0x1.a4e76ce8c0e5ep-4, 0x1.12358f08ae5bap+0, -0x1.1973c5a611cccp-4, \
+    0x1.0953f419900a7p+0, -0x1.252f438e10c1ep-5, 0x1p+0,               0x0p+0,                \
+    0x1.e608cfd9a47acp-1, 0x1.aa5aa5df25984p-5,  0x1.ca4b31f026aap-1,  0x1.c5e53aa362eb4p-4,  \
+    0x1.b2036576afce6p-1, 0x1.526e57720db08p-3,  0x1.9c2d163a1aa2dp-1, 0x1.bc2860d22477p-3,   \
+    0x1.886e6037841edp-1, 0x1.1058bc8a07ee1p-2,  0x1.767dcf5534862p-1, 0x1.4043057b6ee09p-2, }
+#if defined(__CUDACC__)
+static __device__ __constant__ double lz_logf_tab_dev[32] = LZ_LOGF_TAB_INIT;   // {invc, logc} x 16
+#endif
+static const double lz_logf_tab_host[32] = LZ_LOGF_TAB_INIT;
+
+LZ_HD float lz_logf_exact(float x)
+{
+    const double Ln2 = 0x1.62e42fefa39efp-1;
+    const double P0 = -0x1.00ea348b88334p-2, P1 = 0x1.5575b0be00b6ap-2, P2 = -0x1.ffffef20a4123p-2;
+    const uint32_t OFF = 0x3f330000u;
+#if defined(__CUDA_ARCH__)
+    uint32_t ix = __float_as_uint(x);
+#else
+    uint32_t ix;
+    memcpy(&ix, &x, 4);
+#endif
+    if (ix == 0x3f800000u) return 0.0f;
+    if (ix - 0x00800000u >= 0x7f800000u - 0x00800000u) {   // zero, subnormal, inf (negative / NaN are not inputs here)
+        if (ix * 2 == 0) return -__builtin_huge_valf();
+        if (ix == 0x7f800000u) return x;
+        float xs = x * 0x1p23f;                             // subnormal: normalise
+#if defined(__CUDA_ARCH__)
+        ix = __float_as_uint(xs);
+#else
+        memcpy(&ix, &xs, 4);
+#endif
+        ix -= 23u << 23;
+    }
+    const uint32_t tmp = ix - OFF;
+    const int i = (int)((tmp >> (23 - 4)) % 16);
+    const int k = (int32_t)tmp >> 23;
+    const uint32_t iz = ix - (tmp & 0xff800000u);
+#if defined(__CUDA_ARCH__)
+    const double invc = lz_logf_tab_dev[2 * i], logc = lz_logf_tab_dev[2 * i + 1];
+    const double z = (double)__uint_as_float(iz);
+    const double r = __fma_rn(z, invc, -1.0);
+    const double y0 = __fma_rn((double)k, Ln2, logc);
+    const double r2 = __dmul_rn(r, r);
+    double y = __fma_rn(P1, r, P2);
+    y = __fma_rn(P0, r2, y);
+    y = __fma_rn(y, r2, __dadd_rn(y0, r));
+    return __double2float_rn(y);
+#else
+    const double invc = lz_logf_tab_host[2 * i], logc = lz_logf_tab_host[2 * i + 1];
+    float zf;
+    memcpy(&zf, &iz, 4);
+    const double z = (double)zf;
+    const double r = fma(z, invc, -1.0);
+    const double y0 = fma((double)k, Ln2, logc);
+    const double r2 = r * r;
+    double y = fma(P1, r, P2);
+    y = fma(P0, r2, y);
+    y = fma(y, r2, y0 + r);
+    return (float)y;
+#endif
+}

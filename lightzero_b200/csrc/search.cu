@@ -33,6 +33,10 @@ struct lz_search {
     int32_t *d_true_action;
     float *d_reuse_value;
     cudaGraphExec_t exec_reuse;
+    // Gumbel MuZero search graph: captured for one discount (baked into the kernel arguments); the tree generation covers S and m
+    cudaGraphExec_t exec_gumbel;
+    unsigned long long gen_model_gumbel, gen_tree_gumbel;
+    float discount_gumbel;
     cudaGraphExec_t exec[2];     // [deterministic]
     unsigned long long gen_model[3], gen_tree[3];   // model / tree generation each graph (exec[0], exec[1], exec_reuse) was captured at
     cudaStream_t capture_stream; // library-owned: the caller's stream may be the legacy default stream,
@@ -172,6 +176,31 @@ static int enqueue_search_reuse(lz_search *q, cudaStream_t s)
     return LZ_OK;
 }
 
+// GumbelMuZeroMCTSCtree.search (mcts_ctree.py:1076-1174): [traverse] + S x [recurrent_inference, backpropagate (+ next traverse)].
+// The network is the multi-launch model_recurrent of the MuZero search (conv tcgen05 / SIMT or MLP); the persistent MuZero kernel
+// (tree_persist.cuh) has no Gumbel descent.
+static int enqueue_search_gumbel(lz_search *q, float discount, cudaStream_t s)
+{
+    int rc;
+    lz_tree *t = q->tree;
+    if ((rc = gumbel_launch_traverse(t, discount, q->d_ix, nullptr, q->d_action, nullptr, nullptr, s))) return rc;
+    for (int sim = 0; sim < q->S; ++sim) {
+        RecIO io;
+        memset(&io, 0, sizeof(io));
+        io.B = q->B; io.latent_base = q->pool; io.ix = q->d_ix; io.slot_stride = q->slot_stride; io.action = q->d_action;
+        io.next_latent = q->pool + (size_t)(sim + 1) * q->slot_stride;
+        io.reward = q->d_reward; io.value = q->d_value; io.policy_logits = q->d_policy;
+        io.skip_scratch = q->d_skip;
+        if ((rc = model_recurrent(q->model, io, s))) return rc;
+        if (sim + 1 < q->S)
+            rc = gumbel_launch_backprop_traverse(t, sim + 1, discount, q->d_reward, q->d_value, q->d_policy, q->d_ix, q->d_action, s);
+        else
+            rc = gumbel_launch_backprop(t, sim + 1, discount, q->d_reward, q->d_value, q->d_policy, s);
+        if (rc) return rc;
+    }
+    return LZ_OK;
+}
+
 static int run_graph(lz_search *q, int deterministic, cudaStream_t s)
 {
     const int d = deterministic ? 1 : 0;
@@ -257,6 +286,7 @@ int lz_search_destroy(lz_search *q)
     cudaFree(q->hpool); cudaFree(q->cpool); cudaFree(q->d_is_reset);
     cudaFree(q->d_true_action); cudaFree(q->d_reuse_value);
     if (q->exec_reuse) cudaGraphExecDestroy(q->exec_reuse);
+    if (q->exec_gumbel) cudaGraphExecDestroy(q->exec_gumbel);
     delete q;
     return LZ_OK;
 }
@@ -350,6 +380,47 @@ int lz_search_run(lz_search *q, const float *d_latent_roots, int deterministic, 
     if (d_latent_roots && d_latent_roots != q->pool)
         LZ_CUDA_CHECK(cudaMemcpyAsync(q->pool, d_latent_roots, q->slot_stride * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)s));
     return run_graph(q, deterministic, (cudaStream_t)s);
+}
+
+int lz_search_run_gumbel(lz_search *q, const float *d_latent_roots, float discount, lz_stream s_)
+{
+    LZ_REQUIRE(q, LZ_EINVAL, "lz_search_run_gumbel: null search");
+    LZ_REQUIRE(!q->hpool, LZ_EINVAL, "lz_search_run_gumbel: Gumbel MuZero runs on MuZero models, not EfficientZero");
+    lz_tree *t = q->tree;
+    LZ_REQUIRE(t->gumbel, LZ_ESTATE, "lz_search_run_gumbel: tree is not in Gumbel mode (lz_tree_set_gumbel)");
+    LZ_REQUIRE(t->gp.S == q->S, LZ_EINVAL, "lz_search_run_gumbel: tree set for num_simulations=%d, search created for %d", t->gp.S, q->S);
+    LZ_REQUIRE(t->prepared, LZ_ESTATE, "lz_search_run_gumbel: roots not prepared (call lz_tree_prepare_gumbel first)");
+    LZ_REQUIRE(t->gumbel_traversals == 0, LZ_ESTATE, "lz_search_run_gumbel: %d traverses since prepare (prepare again)", t->gumbel_traversals);
+    cudaStream_t s = (cudaStream_t)s_;
+    if (d_latent_roots && d_latent_roots != q->pool)
+        LZ_CUDA_CHECK(cudaMemcpyAsync(q->pool, d_latent_roots, q->slot_stride * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    if (q->exec_gumbel && (q->gen_model_gumbel != q->model->generation || q->gen_tree_gumbel != t->generation ||
+                           q->discount_gumbel != discount)) {
+        cudaGraphExecDestroy(q->exec_gumbel);
+        q->exec_gumbel = nullptr;
+    }
+    if (!q->exec_gumbel) {
+        q->gen_model_gumbel = q->model->generation;
+        q->gen_tree_gumbel = t->generation;
+        q->discount_gumbel = discount;
+        cudaGraph_t graph = nullptr;
+        if (!q->capture_stream) LZ_CUDA_CHECK(cudaStreamCreateWithFlags(&q->capture_stream, cudaStreamNonBlocking));
+        LZ_CUDA_CHECK(cudaStreamBeginCapture(q->capture_stream, cudaStreamCaptureModeThreadLocal));
+        int rc = enqueue_search_gumbel(q, discount, q->capture_stream);
+        cudaError_t e = cudaStreamEndCapture(q->capture_stream, &graph);
+        if (rc != LZ_OK) { if (graph) cudaGraphDestroy(graph); q->exec_gumbel = nullptr; return rc; }
+        if (e != cudaSuccess) { set_error("cudaStreamEndCapture failed: %s", cudaGetErrorString(e)); return LZ_ECUDA; }
+        size_t n = 0;
+        LZ_CUDA_CHECK(cudaGraphGetNodes(graph, nullptr, &n));
+        q->num_kernels = (int)n;
+        e = cudaGraphInstantiate(&q->exec_gumbel, graph, 0);
+        cudaGraphDestroy(graph);
+        if (e != cudaSuccess) { q->exec_gumbel = nullptr; set_error("cudaGraphInstantiate failed: %s", cudaGetErrorString(e)); return LZ_ECUDA; }
+    }
+    LZ_CUDA_CHECK(cudaGraphLaunch(q->exec_gumbel, s));
+    count_launch(q->num_kernels);
+    t->gumbel_traversals = q->S;
+    return LZ_OK;
 }
 
 static int collect_device(lz_search *q, const float *d_obs, const uint8_t *d_obs_u8, const uint8_t *d_mask, const float *d_noise,

@@ -408,6 +408,7 @@ int lz_tree_create(int B, int A, int max_sims, lz_tree **out)
 int lz_tree_destroy(lz_tree *t)
 {
     if (!t) return LZ_OK;
+    gumbel_free(t);
     cudaFree(t->alloc_base);
     delete t;
     return LZ_OK;

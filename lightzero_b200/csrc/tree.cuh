@@ -431,6 +431,16 @@ __device__ __forceinline__ void tree_backprop(const TreeParams &p, int b, int la
     __syncwarp();
 }
 
+// Gumbel MuZero mode (ctree_gumbel_muzero, gumbel.cu).  Allocated by lz_tree_set_gumbel only, so the MuZero / EfficientZero
+// layouts and kernels are untouched; the descent and back-up reuse the node blocks, path storage and expand_block above.
+struct GumbelParams {
+    int S, m;                    // num_simulations, max_num_considered_actions
+    float *raw_value;            // [B][N] value the node was expanded with (the root's from prepare)
+    const float *gumbel;         // [A] 10 * extreme_value(0, 1) draws of std::mt19937(0); a root uses its first nlegal entries
+    const int *visit_row;        // [S] get_sequence_of_considered_visits(min(m, S), S)
+    const int *minus_one;        // [B] all -1: the back-up's to_play (no two-player sign flip, cnode.cpp:605-631)
+};
+
 }  // namespace lz
 
 // ---- internal C++ launch API shared by tree.cu and search.cu ----
@@ -443,6 +453,11 @@ struct lz_tree {
     unsigned long long generation;   // bumped whenever TreeParams values that captured graphs bake in change (set_params / set_ez)
     bool pdl;                    // launch tree kernels with programmatic stream serialization (set by the search graph)
     void *alloc_base;
+    // Gumbel mode (lz_tree_set_gumbel): device tables + the number of traverses since the last prepare (checked on the host)
+    bool gumbel;
+    lz::GumbelParams gp;
+    void *gumbel_alloc;
+    int gumbel_traversals;
 };
 
 namespace lz {
@@ -463,4 +478,13 @@ int tree_launch_backprop_reuse(lz_tree *t, int latent_index, const float *d_rewa
 int tree_launch_backprop_traverse_reuse(lz_tree *t, int latent_index, const float *d_reward, const float *d_value, const float *d_logits,
                                         const int32_t *d_true_action, const float *d_reuse_value, int32_t *d_ix_net, int32_t *d_action,
                                         cudaStream_t s);
+// Gumbel MuZero (gumbel.cu)
+int gumbel_launch_traverse(lz_tree *t, float discount, int32_t *d_ix, int32_t *d_iy, int32_t *d_action, int32_t *d_len,
+                           int32_t *d_vtp, cudaStream_t s);
+int gumbel_launch_backprop(lz_tree *t, int latent_index, float discount, const float *d_reward, const float *d_value,
+                           const float *d_logits, cudaStream_t s);
+// fused: backup of simulation (latent_index - 1) followed by the descent of the next simulation
+int gumbel_launch_backprop_traverse(lz_tree *t, int latent_index, float discount, const float *d_reward, const float *d_value,
+                                    const float *d_logits, int32_t *d_ix, int32_t *d_action, cudaStream_t s);
+void gumbel_free(lz_tree *t);
 }  // namespace lz

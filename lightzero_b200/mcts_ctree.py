@@ -20,7 +20,7 @@ from typing import Any, List, Optional, Union
 import numpy as np
 import torch
 
-from . import cabi, ez_tree, mz_tree
+from . import cabi, ez_tree, gmz_tree, mz_tree
 from .efficientzero_model import EfficientZeroModel
 from .muzero_model import MuZeroModel
 from .muzero_model_mlp import MuZeroModelMLP
@@ -169,18 +169,24 @@ class MuZeroMCTSCtree(object):
             if hasattr(model, "eval"):
                 model.eval()
             for sim in range(S):
-                cabi.check(t.lib.lz_tree_traverse(t.h, int(self.deterministic), t.ix.data_ptr(), t.iy.data_ptr(),
-                                                  t.action.data_ptr(), t.search_len.data_ptr(), t.vtp.data_ptr(),
-                                                  cabi.stream_ptr()), "lz_tree_traverse")
+                self._traverse(t)
                 latent_states = pool[t.ix.long(), rows]                       # mcts_ctree.py:323-324 on device
                 out = model.recurrent_inference(latent_states, t.action.long())
                 pool[sim + 1] = out.latent_state
                 value = self._inv(out.value).reshape(-1).contiguous()        # :349 (value support)
                 reward = self._inv_reward(out.reward).reshape(-1).contiguous()      # :350 (reward support)
                 pol = out.policy_logits.to(torch.float32).contiguous()
-                cabi.check(t.lib.lz_tree_backpropagate(t.h, sim + 1, reward.data_ptr(), value.data_ptr(),
-                                                       pol.data_ptr(), None, cabi.stream_ptr()),
-                           "lz_tree_backpropagate")
+                self._backpropagate(t, sim + 1, reward, value, pol)
+
+    # the tree steps of _search_stepwise (GumbelMuZeroMCTSCtree swaps in the Gumbel descent and back-up)
+    def _traverse(self, t):
+        cabi.check(t.lib.lz_tree_traverse(t.h, int(self.deterministic), t.ix.data_ptr(), t.iy.data_ptr(),
+                                          t.action.data_ptr(), t.search_len.data_ptr(), t.vtp.data_ptr(),
+                                          cabi.stream_ptr()), "lz_tree_traverse")
+
+    def _backpropagate(self, t, latent_index, reward, value, pol):
+        cabi.check(t.lib.lz_tree_backpropagate(t.h, latent_index, reward.data_ptr(), value.data_ptr(),
+                                               pol.data_ptr(), None, cabi.stream_ptr()), "lz_tree_backpropagate")
 
 
 class EfficientZeroMCTSCtree(MuZeroMCTSCtree):
@@ -361,3 +367,67 @@ class UniZeroMCTSCtree(MuZeroMCTSCtree):
                 cabi.check(t.lib.lz_tree_backpropagate(t.h, simulation_index + 1, reward.data_ptr(), value.data_ptr(),
                                                        pol.data_ptr(), None, cabi.stream_ptr()), "lz_tree_backpropagate")
         return first_action_latent_map
+
+
+class GumbelMuZeroMCTSCtree(MuZeroMCTSCtree):
+    """Mirror of ``lzero.mcts.tree_search.mcts_ctree.GumbelMuZeroMCTSCtree`` (mcts_ctree.py:1005-1174): same class-level
+    ``config``, ``default_config()``, ``roots(n, legal_actions)`` (``gmz_tree.Roots``) and
+    ``search(roots, model, latent_state_roots, to_play_batch)``; ``num_simulations``, ``max_num_considered_actions`` and
+    ``discount_factor`` come from the policy config as in the reference (defaults of gumbel_muzero.py: 4 and 0.997).
+
+    With a ``lightzero_b200`` MuZeroModel / MuZeroModelMLP the whole search is one CUDA-graph launch (``lz_search_run_gumbel``);
+    any other model object is driven step-wise around the device trees.  Root choice is sequential halving over the fixed
+    Gumbel draw and interior choice the completed-Q improved policy: no random numbers, so both modes reproduce the reference
+    tree bit for bit on the same network outputs."""
+
+    # mcts_ctree.py:1018-1027
+    config = dict(
+        num_simulations=50,
+        root_dirichlet_alpha=0.3,
+        root_noise_weight=0.25,
+        value_delta_max=0.01,
+    )
+
+    def __init__(self, cfg=None) -> None:
+        super().__init__(cfg)
+        self._cfg.setdefault("max_num_considered_actions", 4)
+        self._cfg.setdefault("env_type", "not_board_games")
+
+    @classmethod
+    def roots(cls, active_collect_env_num: int, legal_actions: List[Any]) -> "gmz_tree.Roots":
+        """mcts_ctree.py:1062-1074"""
+        return gmz_tree.Roots(active_collect_env_num, legal_actions)
+
+    def _gumbel_params(self):
+        return int(self._cfg.num_simulations), int(self._cfg.max_num_considered_actions)
+
+    def search(self, roots: "gmz_tree.Roots", model, latent_state_roots, to_play_batch: Union[int, List[Any]]) -> None:
+        """mcts_ctree.py:1076-1174.  ``latent_state_roots``: np.ndarray or CUDA tensor [B, ...]."""
+        S, m = self._gumbel_params()
+        roots._materialize(S, (S, m))        # reset + Gumbel tables + prepare on the device
+        t = roots._tree
+        dev = roots.device
+        if isinstance(latent_state_roots, torch.Tensor):
+            lat = latent_state_roots.to(dev, torch.float32, non_blocking=True).contiguous()
+        else:
+            lat = torch.from_numpy(np.ascontiguousarray(latent_state_roots, dtype=np.float32)).to(dev, non_blocking=True)
+        if isinstance(model, EfficientZeroModel):
+            raise TypeError("GumbelMuZeroMCTSCtree.search: Gumbel MuZero runs on MuZero models, not an EfficientZeroModel")
+        if isinstance(model, (MuZeroModel, MuZeroModelMLP)):
+            q = t.search_for(model, S)
+            with torch.cuda.device(dev):
+                cabi.check(t.lib.lz_search_run_gumbel(q, lat.data_ptr(), float(self._cfg.discount_factor), cabi.stream_ptr()),
+                           "lz_search_run_gumbel")
+            self.last_num_kernels = t.lib.lz_search_num_kernels(q)
+            return
+        self._search_stepwise(roots, model, lat, S)
+
+    def _traverse(self, t):
+        cabi.check(t.lib.lz_tree_traverse_gumbel(t.h, float(self._cfg.discount_factor), t.ix.data_ptr(), t.iy.data_ptr(),
+                                                 t.action.data_ptr(), t.search_len.data_ptr(), t.vtp.data_ptr(),
+                                                 cabi.stream_ptr()), "lz_tree_traverse_gumbel")
+
+    def _backpropagate(self, t, latent_index, reward, value, pol):
+        cabi.check(t.lib.lz_tree_backpropagate_gumbel(t.h, latent_index, float(self._cfg.discount_factor), reward.data_ptr(),
+                                                      value.data_ptr(), pol.data_ptr(), cabi.stream_ptr()),
+                   "lz_tree_backpropagate_gumbel")

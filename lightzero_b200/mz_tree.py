@@ -285,8 +285,12 @@ class Roots:
                     dn = torch.from_numpy(nl).to(self.device)
                     cabi.check(t.lib.lz_tree_reset(t.h, dl.data_ptr(), dn.data_ptr(), s), "lz_tree_reset")
                     self._keep = (dl, dn)
-            cabi.check(t.lib.lz_tree_prepare(t.h, p["logits"].data_ptr(), cabi.ptr(p["noise"]), p["w"],
-                                             cabi.ptr(p["rewards"]), cabi.ptr(p["to_play"]), s), "lz_tree_prepare")
+            self._prepare_tree(t, p, s)
+
+    def _prepare_tree(self, t: TreeHandle, p: dict, s):
+        """Expands the roots of the freshly reset tree from the staged prepare() arguments."""
+        cabi.check(t.lib.lz_tree_prepare(t.h, p["logits"].data_ptr(), cabi.ptr(p["noise"]), p["w"],
+                                         cabi.ptr(p["rewards"]), cabi.ptr(p["to_play"]), s), "lz_tree_prepare")
 
 
 def batch_traverse(roots: Roots, pb_c_base: int, pb_c_init: float, discount_factor: float,
